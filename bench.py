@@ -6,7 +6,7 @@ per GPU (left: 100 chunks of 1M rows; right: chunks of 999,983 rows so the execu
 iteration sees misaligned chunk boundaries, arrow/compute/executor.go:757-863), one contiguous
 preallocated output (executor.go:598-623).  A "step" is one Add over the whole column.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 ONE JSON line on rank 0 (contract in the task statement):
   value     rows/s, whole job (all ranks), kernels timed with CUDA events on device-resident
@@ -387,6 +387,19 @@ def c3_pipeline(N, h_vals, h_out, d_vals, d_out, rows, rank, Event, barrier, max
             "note": "Greater(int64, 89) + Filter fused (ag_filter_compare_scalar_dev) on the resident column; wall clock incl. the count readback and the D2H of the selected rows"}
 
 
+DUMP_NAME = "add_f64_chunked_output"
+DUMP_ROWS = 1 << 20   # 8 MB of float64
+DUMP_SEED = 0xD0770
+
+
+def dump_outputs(out_dir, out):
+    """Rows of the Add output sampled without replacement by a fixed seed, so two builds given the same arguments
+    write comparable files."""
+    rows = np.sort(np.random.default_rng(DUMP_SEED).choice(out.size, min(DUMP_ROWS, out.size), replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, DUMP_NAME + ".npy"), out[rows])
+
+
 # ------------------------------------------------------------------ our arm ---------------
 def main():
     ap = argparse.ArgumentParser()
@@ -400,7 +413,11 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-full-configs", action="store_true", help="skip BASELINE configs 4/5 at 1B rows")
     ap.add_argument("--full-rows", type=int, default=1_000_000_000, help="total rows of configs 4/5 (split over the ranks)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write rank 0's Add output of the last "
+                    f"step as DIR/{DUMP_NAME}.npy (float64, a fixed seeded sample of {DUMP_ROWS} rows, ascending)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     _claim_stdout()
     if args.impl == "reference":
         run_reference_arm(args)
@@ -433,7 +450,7 @@ def main():
         except Exception as e:  # no libnccl.so.2 the product can dlopen: the mailbox form still runs
             print(f"rank {rank}: NCCL attach failed: {e}", file=sys.stderr)
     rows = args.rows
-    W, K = max(args.warmup, 3), max(args.steps, 1)
+    W, K = max(args.warmup, 3), args.steps
     peak, peak_kind = peaks()
 
     def barrier():
@@ -488,6 +505,8 @@ def main():
     l0 = N.raw().ag_kernel_launch_count()
     ms_chunked = timed(add_step, W, K)
     launches_timed = (N.raw().ag_kernel_launch_count() - l0) * K // (W + K)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dout.to_numpy(np.float64, rows))
     ms_per_span = timed(add_step_per_span, 3, max(3, K // 4))
     ms_contig = timed(lambda: N.call("ag_arith_binary_dev", N.FLOAT64, N.OP_ADD_CHECKED, N.SHAPE_AA, dl.ptr, dr.ptr, dout.ptr, rows, None), W, K)
 

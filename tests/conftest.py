@@ -19,20 +19,30 @@ def cpu():
     return oracle.cpu()
 
 
-@pytest.fixture(scope="session")
-def ref():
-    """The reference's own AVX2/SSE4 loops (oracle/_ref); skip if never built."""
+@pytest.fixture
+def ref(request, cpu, isa):
+    """The reference's own AVX2/SSE4 loops: oracle/_ref where it was built, otherwise their recorded
+    replay (tests/ref_replay.py)."""
+    import ref_replay
     from oracle import oracle
     lib = oracle.ref()
+    key = ref_replay.key_of(request.node)
     if lib is None:
-        pytest.skip("oracle/_ref/libarrowgo_ref.so not built (needs /root/reference)")
-    return lib
+        replay = ref_replay.Replay(key, cpu)
+        yield replay
+        replay.done()
+    elif os.environ.get(ref_replay.RECORD_ENV):
+        yield ref_replay.Recorder(lib, key, cpu, isa)
+    else:
+        yield lib
 
 
 @pytest.fixture(scope="session")
 def isa():
+    """The ISA whose reference loops the tests compare against: the host's, or the recorded one."""
+    import ref_replay
     from oracle import oracle
-    return oracle.host_isa()
+    return oracle.host_isa() if oracle.ref() is not None else ref_replay.table()["isa"]
 
 
 @pytest.fixture(scope="session")
