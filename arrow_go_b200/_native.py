@@ -171,6 +171,8 @@ _SIGS = {
     "ag_is_in_dev": [_i, _p, _p, _i64, _i64, _p, _p, _i64, _i64, _i, _p, _p, _p, _p],
     "ag_unique": [_i, _p, _p, _i64, _i64, _p, _p, _pi64, _pi64],
     "ag_unique_dev": [_i, _p, _p, _i64, _i64, _p, _p, _i64, _p, _p],
+    "ag_dictionary_encode": [_i, _p, _p, _i64, _i64, _i, _p, _p, _p, _p, _pi64, _pi64],
+    "ag_dictionary_encode_dev": [_i, _p, _p, _i64, _i64, _i, _p, _p, _p, _p, _i64, _p, _p],
     "ag_sort_indices": [_i, _p, _p, _i64, _i64, _i, _i, _p, _pi64, _pi64],
     "ag_sort_indices_dev": [_i, _p, _p, _i64, _i64, _i, _i, _p, _pi64, _pi64, _p],
     "ag_parquet_unpack32": [_p, _p, _i64, _i, _pi64],

@@ -23,6 +23,7 @@ HOST_LIB_PATH = os.path.join(_HERE, "lib", "libarrowgpu_host.so")
 
 # arrow.Type ids
 NA, BOOL, UINT8, INT8, UINT16, INT16, UINT32, INT32, UINT64, INT64, FLOAT16, FLOAT32, FLOAT64 = range(13)
+DICTIONARY = 29  # int32 indices + a dictionary (Datum.dictionary()); to_numpy() gives the indices
 NP_OF = {UINT8: np.uint8, INT8: np.int8, UINT16: np.uint16, INT16: np.int16, UINT32: np.uint32, INT32: np.int32,
          UINT64: np.uint64, INT64: np.int64, FLOAT32: np.float32, FLOAT64: np.float64}
 TYPE_OF_NP = {np.dtype(v): k for k, v in NP_OF.items()}
@@ -85,6 +86,8 @@ def lib():
         h.agx_sort_indices.argtypes = [p, i, i, pp]
         h.agx_unique.argtypes = [p, pp]
         h.agx_is_in.argtypes = [p, p, i, pp]
+        h.agx_dictionary_encode.argtypes = [p, i, pp]
+        h.agx_dictionary.argtypes = [p, pp]
         _lib = h
     return _lib
 
@@ -141,12 +144,19 @@ class Datum:
             res.append(Datum(out))
         return res
 
+    def dictionary(self):
+        """The dictionary of a dictionary array (or of one chunk of a dictionary-encoded chunked array)."""
+        out = C.c_void_p()
+        _check(lib().agx_dictionary(self._h, C.byref(out)))
+        return Datum(out)
+
     def to_numpy(self):
-        """(values, valid_bools, null_count) of an Array, or the concatenation over a Chunked."""
+        """(values, valid_bools, null_count) of an Array, or the concatenation over a Chunked.  A dictionary array
+        gives its int32 indices."""
         if self.kind == KIND_CHUNKED:
             parts = [c.to_numpy() for c in self.chunks()]
             if not parts:
-                dt = np.bool_ if self.type == BOOL else NP_OF[self.type]
+                dt = np.bool_ if self.type == BOOL else _np_of(self.type)
                 return np.zeros(0, dtype=dt), np.zeros(0, dtype=bool), 0
             return np.concatenate([p[0] for p in parts]), np.concatenate([p[1] for p in parts]), sum(p[2] for p in parts)
         n = len(self)
@@ -157,7 +167,7 @@ class Datum:
             _check(lib().agx_array_to_host(self._h, raw.ctypes.data, vbytes.ctypes.data, C.byref(nulls)))
             vals = np.unpackbits(raw, bitorder="little")[:n].astype(bool)
         else:
-            vals = np.zeros(n, dtype=NP_OF[self.type])
+            vals = np.zeros(n, dtype=_np_of(self.type))
             _check(lib().agx_array_to_host(self._h, vals.ctypes.data, vbytes.ctypes.data, C.byref(nulls)))
         valid = np.unpackbits(vbytes, bitorder="little")[:n].astype(bool)
         return vals, valid, int(nulls.value)
@@ -169,6 +179,10 @@ class Datum:
     @property
     def null_count(self):
         return self.to_numpy()[2]
+
+
+def _np_of(type_id):
+    return np.int32 if type_id == DICTIONARY else NP_OF[type_id]
 
 
 class Array:
@@ -328,6 +342,18 @@ def IsIn(values, value_set, null_behavior=NULL_MATCH):
     """compute.IsIn(ctx, SetOptions{ValueSet, NullBehavior}, values) (arrow/compute/scalar_set_lookup.go)."""
     out = C.c_void_p()
     _check(lib().agx_is_in(values._h, value_set._h, int(null_behavior), C.byref(out)))
+    return Datum(out)
+
+
+NULL_ENCODING_MASK, NULL_ENCODING_ENCODE = 0, 1
+
+
+def DictionaryEncode(values, null_encoding=NULL_ENCODING_MASK):
+    """compute.DictionaryEncode(ctx, DictionaryEncodeOptions{NullEncoding}, values) (arrow/compute/vector_hash.go):
+    a dictionary array of int32 indices whose dictionary holds the distinct values in order of first appearance.  A
+    chunked input gives a chunked output with the same chunk lengths and one shared dictionary."""
+    out = C.c_void_p()
+    _check(lib().agx_dictionary_encode(values._h, int(null_encoding), C.byref(out)))
     return Datum(out)
 
 

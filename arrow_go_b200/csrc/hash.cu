@@ -22,7 +22,15 @@
 //           the call stays stream-ordered.  Each warp also keeps the last keys it met in a small shared-memory cache:
 //           a key met at a lower row of the same warp cannot be a first appearance, so low-cardinality columns
 //           (the usual dictionary-encoding case) hardly touch the table at all.
-// Roofline: HBM, 8 B/row read once per pass (is_in: one pass; unique: insert + mark + compaction).
+//   dictionary_encode (kernels/vector_hash.go:144-241 dictionaryEncodeAction over doAppendNumeric :359-385) follows
+//           the same table policy as unique (ag_unique_set_policy) and the same insert + mark passes; then the
+//           first rows are ranked (an exclusive scan of popc(keep) per tile), the finalize pass writes each distinct
+//           value to dict[rank] and stores the rank in the slot's spare word, and one streaming pass writes an int32
+//           index per row (one probe returns key + first row + rank in a 16-byte load; a per-warp (key, rank)
+//           cache keeps low-cardinality columns off the table).  Ranks are positions of first rows, so the output
+//           does not depend on the order in which threads reached the table.
+// Roofline: HBM, 8 B/row read once per pass (is_in: one pass; unique: insert + mark + compaction; dictionary_encode:
+// insert + mark + encode, which also writes 4 B/row).
 #include "common.cuh"
 
 namespace ag {
@@ -38,7 +46,8 @@ constexpr unsigned long long kEmptyKey = 0xffffffffffffffffull;
 constexpr unsigned kNoRow = 0xffffffffu;
 constexpr unsigned kNoCap = 0xffffffffu;
 
-struct alignas(16) Slot { unsigned long long key; unsigned first; unsigned pad; };
+// `rank`: unused by is_in / unique; dictionary_encode's finalize pass stores the key's dictionary position there
+struct alignas(16) Slot { unsigned long long key; unsigned first; unsigned rank; };
 
 struct HashTable {
   Slot* slots;                // cleared to all-ones: key = kEmptyKey (free), first = kNoRow
@@ -46,7 +55,8 @@ struct HashTable {
   int shift;                  // 64 - log2(slots)
   unsigned cap;               // distinct keys after which an insert raises special[3] and stops (kNoCap: never)
   unsigned* special;          // [0] lowest row whose key is the all-ones pattern (cannot live in `slots`), [1] lowest NULL row,
-                              // [2] distinct keys inserted, [3] overflow word (0xffffffff after the clear = not raised)
+                              // [2] distinct keys inserted, [3] overflow word (0xffffffff after the clear = not raised),
+                              // [4] / [5] dictionary_encode: ranks of the all-ones key / of the null entry
 };
 
 // multiplicative (Fibonacci) hash of the folded key, forced even: every probe sequence starts on an aligned slot pair
@@ -297,13 +307,9 @@ is_in_kernel(const V* __restrict__ vals, const uint8_t* __restrict__ valid, int6
   if (lane < kHUnroll && nulls && null_count) atomicAdd(null_count, nulls);
 }
 
-// unique: row i is kept iff it is the first row of its key (or the first null row).  `big` is the full-size table of an
-// overflowed call (slots == NULL when the call has only one table).
-template <typename V>
-__global__ void __launch_bounds__(kHThreads)
-unique_mark_kernel(const V* __restrict__ vals, const uint8_t* __restrict__ valid, int64_t off, int64_t n, const HashTable small_t,
-                   const HashTable big_t, uint32_t* __restrict__ keep) {
-  __shared__ unsigned long long s_cache[kHWarps][kWarpCacheSlots];
+// the table that holds the complete result: `big` is the full-size table of an overflowed call (slots == NULL when the
+// call has only one table)
+__device__ __forceinline__ HashTable complete_table(const HashTable& small_t, const HashTable& big_t) {
   const bool use_big = big_t.slots && overflowed(small_t);
   HashTable t;
   t.slots = use_big ? big_t.slots : small_t.slots;
@@ -311,6 +317,17 @@ unique_mark_kernel(const V* __restrict__ vals, const uint8_t* __restrict__ valid
   t.shift = use_big ? big_t.shift : small_t.shift;
   t.cap = kNoCap;
   t.special = use_big ? big_t.special : small_t.special;
+  return t;
+}
+
+// unique: row i is kept iff it is the first row of its key (or, with `count_null`, the first null row; dictionary_encode's
+// mask mode gives nulls no dictionary entry).
+template <typename V>
+__global__ void __launch_bounds__(kHThreads)
+unique_mark_kernel(const V* __restrict__ vals, const uint8_t* __restrict__ valid, int64_t off, int64_t n, const HashTable small_t,
+                   const HashTable big_t, bool count_null, uint32_t* __restrict__ keep) {
+  __shared__ unsigned long long s_cache[kHWarps][kWarpCacheSlots];
+  const HashTable t = complete_table(small_t, big_t);
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   unsigned long long* cache = s_cache[warp];
   for (int i = lane; i < kWarpCacheSlots; i += 32) cache[i] = kEmptyKey;
@@ -343,7 +360,7 @@ unique_mark_kernel(const V* __restrict__ vals, const uint8_t* __restrict__ valid
       const int cs = warp_cache_slot(key);
       const bool ones = sizeof(V) == 8 && key == kEmptyKey;
       bool kp = false;
-      if (kind[k] == 2) kp = first_null == row;
+      if (kind[k] == 2) kp = count_null && first_null == row;
       else if (kind[k] == 1 && ones) kp = first_ones == row;
       const bool go = kind[k] == 1 && !ones && cache[cs] != key;   // a cached key sits at a lower row: not first
       __syncwarp();
@@ -447,32 +464,49 @@ ag_status is_in_dev(int bit_width, const void* vals, const uint8_t* valid, int64
 static std::atomic<long long> g_unique_small_rows{1ll << 21};
 static std::atomic<long long> g_unique_small_slots{1ll << 22};
 
+// Insert pass of unique / dictionary_encode: every key's lowest row, in the small table or (after an overflow, decided
+// on the device) in the full-size one, plus the first-row bitmap `keep` (n/32 words) for the mark pass.
+struct FirstRowTables {
+  TableMem small_t, big_t;
+  uint32_t* keep = nullptr;
+  template <typename V>
+  ag_status build(const V* v, const uint8_t* valid, int64_t off, int64_t n, int grid, cudaStream_t st) {
+    const bool two = n > g_unique_small_rows.load(std::memory_order_relaxed);
+    const unsigned long long small_slots = (unsigned long long)g_unique_small_slots.load(std::memory_order_relaxed);
+    if (two) AG_TRY(small_t.alloc(0, small_slots, (unsigned)(small_slots / 2), st));
+    else AG_TRY(small_t.alloc(n, 1024, kNoCap, st));
+    AG_TRY(small_t.clear(st));
+    if (two) AG_TRY(big_t.alloc(n, 1024, kNoCap, st));
+    AG_TRY(dev_alloc_async((void**)&keep, (size_t)((n + 31) / 32) * 4 + 64, st));
+    hash_insert_kernel<V><<<grid, kHThreads, 0, st>>>(v, valid, off, n, small_t.t, nullptr);
+    AG_TRY(check_launch("hash_insert_kernel"));
+    if (two) {
+      const unsigned* raised = small_t.t.special + 3;
+      AG_TRY(big_t.clear(st, raised));
+      hash_insert_kernel<V><<<grid, kHThreads, 0, st>>>(v, valid, off, n, big_t.t, raised);
+      AG_TRY(check_launch("hash_insert_kernel"));
+    }
+    return AG_OK;
+  }
+  void release(cudaStream_t st) {
+    if (keep) cudaFreeAsync(keep, st);
+    keep = nullptr;
+    small_t.release(st);
+    big_t.release(st);
+  }
+};
+
 template <typename V>
 static ag_status unique_t(int bit_width, const void* vals, const uint8_t* valid, int64_t off, int64_t n, void* out, uint8_t* out_valid,
                           int64_t capacity, int64_t* d_out_len, cudaStream_t st) {
-  const bool two = n > g_unique_small_rows.load(std::memory_order_relaxed);
-  const unsigned long long small_slots = (unsigned long long)g_unique_small_slots.load(std::memory_order_relaxed);
-  TableMem small_t, big_t;
-  uint32_t* keep = nullptr;
+  FirstRowTables tabs;
   ag_status rc = AG_OK;
   do {
-    if (two) rc = small_t.alloc(0, small_slots, (unsigned)(small_slots / 2), st);
-    else rc = small_t.alloc(n, 1024, kNoCap, st);
-    if (rc != AG_OK) break;
-    if ((rc = small_t.clear(st)) != AG_OK) break;
-    if (two && (rc = big_t.alloc(n, 1024, kNoCap, st)) != AG_OK) break;
-    if ((rc = dev_alloc_async((void**)&keep, (size_t)((n + 31) / 32) * 4 + 64, st)) != AG_OK) break;
     const V* v = reinterpret_cast<const V*>(vals);
     const int grid = grid_for(n, kHThreads * kHUnroll, 8);
-    hash_insert_kernel<V><<<grid, kHThreads, 0, st>>>(v, valid, off, n, small_t.t, nullptr);
-    if ((rc = check_launch("hash_insert_kernel")) != AG_OK) break;
-    if (two) {
-      const unsigned* raised = small_t.t.special + 3;
-      if ((rc = big_t.clear(st, raised)) != AG_OK) break;
-      hash_insert_kernel<V><<<grid, kHThreads, 0, st>>>(v, valid, off, n, big_t.t, raised);
-      if ((rc = check_launch("hash_insert_kernel")) != AG_OK) break;
-    }
-    unique_mark_kernel<V><<<grid, kHThreads, 0, st>>>(v, valid, off, n, small_t.t, big_t.t, keep);
+    if ((rc = tabs.build(v, valid, off, n, grid, st)) != AG_OK) break;
+    uint32_t* keep = tabs.keep;
+    unique_mark_kernel<V><<<grid, kHThreads, 0, st>>>(v, valid, off, n, tabs.small_t.t, tabs.big_t.t, true, keep);
     if ((rc = check_launch("unique_mark_kernel")) != AG_OK) break;
     if (out_valid) {
       if (cudaMemsetAsync(out_valid, 0, (size_t)((capacity + 31) / 32) * 4, st) != cudaSuccess) { rc = cuda_fail(cudaGetLastError(), "memset", __FILE__, __LINE__); break; }
@@ -480,9 +514,7 @@ static ag_status unique_t(int bit_width, const void* vals, const uint8_t* valid,
     rc = filter_primitive_dev(bit_width, vals, valid, off, reinterpret_cast<const uint8_t*>(keep), nullptr, 0, n, AG_DROP_NULLS, out, out_valid,
                               capacity, d_out_len, st);
   } while (0);
-  if (keep) cudaFreeAsync(keep, st);
-  small_t.release(st);
-  big_t.release(st);
+  tabs.release(st);
   return rc;
 }
 
@@ -500,6 +532,255 @@ ag_status unique_dev(int bit_width, const void* vals, const uint8_t* valid, int6
     case 32: return unique_t<uint32_t>(bit_width, vals, valid, off, n, out, out_valid, capacity, d_out_len, st);
     case 64: return unique_t<unsigned long long>(bit_width, vals, valid, off, n, out, out_valid, capacity, d_out_len, st);
     default: AG_FAIL(AG_ERR_NOT_IMPLEMENTED, "unique: fixed-width values of 1/2/4/8 bytes only (got %d bits)", bit_width);
+  }
+}
+
+// ---- dictionary_encode: rank + finalize + encode passes after unique's insert + mark ------------------------------------
+constexpr int kRankWordsPerThread = 8;
+constexpr int kRankTileWords = kHThreads * kRankWordsPerThread;   // keep words (65536 rows) per rank tile
+
+// exclusive prefix of `x` over the block; *total = the block's sum
+template <int kThreads>
+__device__ __forceinline__ unsigned block_exclusive_scan(unsigned x, unsigned* total) {
+  __shared__ unsigned s_warp[kThreads / 32];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  unsigned inc = x;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const unsigned y = __shfl_up_sync(0xffffffffu, inc, o);
+    if (lane >= o) inc += y;
+  }
+  if (lane == 31) s_warp[warp] = inc;
+  __syncthreads();
+  if (warp == 0) {
+    unsigned w = lane < kThreads / 32 ? s_warp[lane] : 0u;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const unsigned y = __shfl_up_sync(0xffffffffu, w, o);
+      if (lane >= o) w += y;
+    }
+    if (lane < kThreads / 32) s_warp[lane] = w;
+  }
+  __syncthreads();
+  const unsigned base = warp ? s_warp[warp - 1] : 0u;
+  *total = s_warp[kThreads / 32 - 1];
+  __syncthreads();   // s_warp is reused by the next call
+  return base + inc - x;
+}
+
+// number of first rows per rank tile
+__global__ void __launch_bounds__(kHThreads)
+dict_rank_count_kernel(const uint32_t* __restrict__ keep, int64_t n_words, unsigned* __restrict__ tile_sums) {
+  const int64_t w0 = (int64_t)blockIdx.x * kRankTileWords + (int64_t)threadIdx.x * kRankWordsPerThread;
+  unsigned c = 0;
+#pragma unroll
+  for (int k = 0; k < kRankWordsPerThread; ++k) c += w0 + k < n_words ? __popc(keep[w0 + k]) : 0u;
+  unsigned total;
+  block_exclusive_scan<kHThreads>(c, &total);
+  if (threadIdx.x == 0) tile_sums[blockIdx.x] = total;
+}
+
+// tile_sums -> exclusive tile offsets (in place); counts[0] = dictionary length
+constexpr int kRankScanThreads = 1024;
+__global__ void __launch_bounds__(kRankScanThreads)
+dict_rank_scan_kernel(unsigned* __restrict__ tile_sums, int64_t tiles, long long* __restrict__ counts) {
+  unsigned carry = 0;
+  for (int64_t b = 0; b < tiles; b += kRankScanThreads) {
+    const int64_t i = b + threadIdx.x;
+    const unsigned x = i < tiles ? tile_sums[i] : 0u;
+    unsigned total;
+    const unsigned ex = block_exclusive_scan<kRankScanThreads>(x, &total);
+    if (i < tiles) tile_sums[i] = carry + ex;
+    carry += total;
+  }
+  if (threadIdx.x == 0) counts[0] = (long long)carry;
+}
+
+// slot of a key that is in the table
+__device__ __forceinline__ Slot* table_slot(const HashTable& t, unsigned long long key) {
+  unsigned long long h = hash_slot(key, t.shift);
+  while (true) {
+    const unsigned long long k = t.slots[h].key;
+    if (k == key) return t.slots + h;
+    if (k == kEmptyKey) return nullptr;
+    h = (h + 1) & t.mask;
+  }
+}
+
+// one lane per first row: dict[rank] = its value, the rank goes to the key's slot (or special[4] / special[5])
+template <typename V>
+__global__ void __launch_bounds__(kHThreads)
+dict_finalize_kernel(const V* __restrict__ vals, const uint8_t* __restrict__ valid, int64_t off, const HashTable small_t,
+                     const HashTable big_t, const uint32_t* __restrict__ keep, int64_t n_words, const unsigned* __restrict__ tile_off,
+                     V* __restrict__ dict, uint32_t* __restrict__ dict_valid, int64_t dict_capacity) {
+  const HashTable t = complete_table(small_t, big_t);
+  const int64_t w0 = (int64_t)blockIdx.x * kRankTileWords + (int64_t)threadIdx.x * kRankWordsPerThread;
+  uint32_t words[kRankWordsPerThread];
+  unsigned c = 0;
+#pragma unroll
+  for (int k = 0; k < kRankWordsPerThread; ++k) {
+    words[k] = w0 + k < n_words ? keep[w0 + k] : 0u;
+    c += __popc(words[k]);
+  }
+  unsigned total;
+  unsigned rank = tile_off[blockIdx.x] + block_exclusive_scan<kHThreads>(c, &total);
+#pragma unroll
+  for (int k = 0; k < kRankWordsPerThread; ++k) {
+    uint32_t bits = words[k];
+    while (bits) {
+      const int64_t row = ((w0 + k) << 5) + (__ffs(bits) - 1);
+      bits &= bits - 1;
+      const bool is_null = valid && !bit_is_set(valid, off + row);
+      const V x = is_null ? V(0) : vals[off + row];
+      if ((int64_t)rank < dict_capacity) {
+        dict[rank] = x;
+        if (is_null && dict_valid) atomicAnd(&dict_valid[rank >> 5], ~(1u << (rank & 31)));
+      }
+      const unsigned long long key = (unsigned long long)x;
+      if (is_null) t.special[5] = rank;
+      else if (sizeof(V) == 8 && key == kEmptyKey) t.special[4] = rank;
+      else table_slot(t, key)->rank = rank;
+      ++rank;
+    }
+  }
+}
+
+// rank of a key that is in the table: key, first row and rank arrive in one 16-byte load
+__device__ __forceinline__ unsigned table_rank(const HashTable& t, unsigned long long key) {
+  unsigned long long h = hash_slot(key, t.shift);
+  while (true) {
+    const ulonglong2 raw = *reinterpret_cast<const ulonglong2*>(t.slots + h);
+    if (raw.x == key) return (unsigned)(raw.y >> 32);
+    if (raw.x == kEmptyKey) return 0u;
+    h = (h + 1) & t.mask;
+  }
+}
+
+// one int32 index per row.  Mask mode: a null row gets index 0 and a cleared validity bit; encode mode: the null entry's
+// rank.  The table is read-only here, so a per-warp cache of (key, rank) pairs is always right.
+template <typename V>
+__global__ void __launch_bounds__(kHThreads)
+dict_encode_kernel(const V* __restrict__ vals, const uint8_t* __restrict__ valid, int64_t off, int64_t n, const HashTable small_t,
+                   const HashTable big_t, bool mask_nulls, int32_t* __restrict__ indices, uint32_t* __restrict__ indices_valid,
+                   unsigned long long* __restrict__ null_count) {
+  __shared__ unsigned long long s_key[kHWarps][kWarpCacheSlots];
+  __shared__ unsigned s_rank[kHWarps][kWarpCacheSlots];
+  const HashTable t = complete_table(small_t, big_t);
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  unsigned long long* ckey = s_key[warp];
+  unsigned* crank = s_rank[warp];
+  for (int i = lane; i < kWarpCacheSlots; i += 32) ckey[i] = kEmptyKey;
+  __syncwarp();
+  const unsigned ones_rank = t.special[4], null_rank = mask_nulls ? 0u : t.special[5];
+  const int64_t n_words = (n + 31) >> 5;
+  const int64_t warp0 = ((int64_t)blockIdx.x * kHThreads + threadIdx.x) >> 5;
+  const int64_t warps = ((int64_t)gridDim.x * kHThreads) >> 5;
+  unsigned long long nulls = 0;
+  for (int64_t w0 = warp0 * kHUnroll; w0 < n_words; w0 += warps * kHUnroll) {
+    V x[kHUnroll];
+    int kind[kHUnroll];                                  // 0 nothing, 1 value, 2 null
+    if (!valid && ((w0 + kHUnroll) << 5) <= n) {
+      const V* __restrict__ p = vals + off + (w0 << 5) + lane;
+#pragma unroll
+      for (int k = 0; k < kHUnroll; ++k) { x[k] = __ldcs(p + 32 * k); kind[k] = 1; }
+    } else {
+#pragma unroll
+      for (int k = 0; k < kHUnroll; ++k) {
+        const int64_t i = ((w0 + k) << 5) + lane;
+        kind[k] = i < n ? ((valid && !bit_is_set(valid, off + i)) ? 2 : 1) : 0;
+        x[k] = kind[k] == 1 ? __ldcs(vals + off + i) : V(0);
+      }
+    }
+#pragma unroll
+    for (int k = 0; k < kHUnroll; ++k) {
+      const int64_t w = w0 + k;
+      if (w >= n_words) break;   // warp-uniform
+      const unsigned long long key = (unsigned long long)x[k];
+      const int cs = warp_cache_slot(key);
+      const bool ones = sizeof(V) == 8 && key == kEmptyKey;
+      unsigned idx = kind[k] == 2 ? null_rank : ones_rank;
+      bool miss = false;
+      if (kind[k] == 1 && !ones) {
+        if (ckey[cs] == key) idx = crank[cs];
+        else miss = true;
+      }
+      __syncwarp();
+      if (miss) { idx = table_rank(t, key); atomicExch(&ckey[cs], key); }   // several lanes may share a slot: one whole key wins
+      __syncwarp();
+      if (miss && ckey[cs] == key) crank[cs] = idx;                        // every lane holding the winning key writes the same rank
+      __syncwarp();
+      if (kind[k] != 0) __stcs(indices + (w << 5) + lane, (int32_t)idx);
+      if (indices_valid) {
+        const uint32_t vbits = __ballot_sync(0xffffffffu, kind[k] == 1 || (kind[k] == 2 && !mask_nulls));
+        if (lane == 0) {
+          indices_valid[w] = vbits;
+          const int64_t rem = n - (w << 5);
+          nulls += __popc(~vbits & (rem >= 32 ? 0xffffffffu : bit_range_mask(0, (int)rem)));
+        }
+      }
+    }
+  }
+  if (lane == 0 && nulls) atomicAdd(null_count, nulls);
+}
+
+template <typename V>
+static ag_status dictionary_encode_t(const void* vals, const uint8_t* valid, int64_t off, int64_t n, int null_encoding, int32_t* indices,
+                                     uint8_t* indices_valid, void* dict, uint8_t* dict_valid, int64_t dict_capacity, int64_t* d_counts,
+                                     cudaStream_t st) {
+  FirstRowTables tabs;
+  unsigned* tile_off = nullptr;
+  ag_status rc = AG_OK;
+  const bool mask_nulls = null_encoding == AG_NULL_ENCODING_MASK;
+  do {
+    const V* v = reinterpret_cast<const V*>(vals);
+    const int grid = grid_for(n, kHThreads * kHUnroll, 8);
+    const int64_t n_words = (n + 31) / 32;
+    const int64_t tiles = (n_words + kRankTileWords - 1) / kRankTileWords;
+    if (cudaMemsetAsync(d_counts, 0, 2 * sizeof(int64_t), st) != cudaSuccess) { rc = cuda_fail(cudaGetLastError(), "memset", __FILE__, __LINE__); break; }
+    if ((rc = tabs.build(v, valid, off, n, grid, st)) != AG_OK) break;
+    if ((rc = dev_alloc_async((void**)&tile_off, (size_t)tiles * 4 + 64, st)) != AG_OK) break;
+    unique_mark_kernel<V><<<grid, kHThreads, 0, st>>>(v, valid, off, n, tabs.small_t.t, tabs.big_t.t, !mask_nulls, tabs.keep);
+    if ((rc = check_launch("unique_mark_kernel")) != AG_OK) break;
+    dict_rank_count_kernel<<<(unsigned)tiles, kHThreads, 0, st>>>(tabs.keep, n_words, tile_off);
+    if ((rc = check_launch("dict_rank_count_kernel")) != AG_OK) break;
+    dict_rank_scan_kernel<<<1, kRankScanThreads, 0, st>>>(tile_off, tiles, reinterpret_cast<long long*>(d_counts));
+    if ((rc = check_launch("dict_rank_scan_kernel")) != AG_OK) break;
+    if (dict_valid && dict_capacity > 0) {
+      if (cudaMemsetAsync(dict_valid, 0xff, (size_t)((dict_capacity + 31) / 32) * 4, st) != cudaSuccess) { rc = cuda_fail(cudaGetLastError(), "memset", __FILE__, __LINE__); break; }
+    }
+    dict_finalize_kernel<V><<<(unsigned)tiles, kHThreads, 0, st>>>(v, valid, off, tabs.small_t.t, tabs.big_t.t, tabs.keep, n_words, tile_off,
+                                                                  reinterpret_cast<V*>(dict), reinterpret_cast<uint32_t*>(dict_valid), dict_capacity);
+    if ((rc = check_launch("dict_finalize_kernel")) != AG_OK) break;
+    dict_encode_kernel<V><<<grid, kHThreads, 0, st>>>(v, valid, off, n, tabs.small_t.t, tabs.big_t.t, mask_nulls, indices,
+                                                      reinterpret_cast<uint32_t*>(indices_valid), reinterpret_cast<unsigned long long*>(d_counts + 1));
+    rc = check_launch("dict_encode_kernel");
+  } while (0);
+  if (tile_off) cudaFreeAsync(tile_off, st);
+  tabs.release(st);
+  return rc;
+}
+
+ag_status dictionary_encode_dev(int bit_width, const void* vals, const uint8_t* valid, int64_t off, int64_t n, int null_encoding, int32_t* indices,
+                                uint8_t* indices_valid, void* dict, uint8_t* dict_valid, int64_t dict_capacity, int64_t* d_counts, cudaStream_t st) {
+  if (n < 0 || off < 0 || dict_capacity < 0) AG_FAIL(AG_ERR_INVALID, "dictionary_encode: negative length, offset or capacity");
+  if (null_encoding != AG_NULL_ENCODING_MASK && null_encoding != AG_NULL_ENCODING_ENCODE)
+    AG_FAIL(AG_ERR_INVALID, "dictionary_encode: invalid null encoding behavior %d", null_encoding);
+  if (!d_counts) AG_FAIL(AG_ERR_INVALID, "dictionary_encode: NULL counts word");
+  if (n == 0) { AG_CUDA_TRY(cudaMemsetAsync(d_counts, 0, 2 * sizeof(int64_t), st)); return AG_OK; }
+  if (!vals || !indices || (!dict && dict_capacity > 0)) AG_FAIL(AG_ERR_INVALID, "dictionary_encode: NULL values / indices / dictionary");
+  if (valid && null_encoding == AG_NULL_ENCODING_MASK && !indices_valid)
+    AG_FAIL(AG_ERR_INVALID, "dictionary_encode: an input with a validity bitmap needs an indices validity bitmap in mask mode");
+  if (valid && null_encoding == AG_NULL_ENCODING_ENCODE && !dict_valid && dict_capacity > 0)
+    AG_FAIL(AG_ERR_INVALID, "dictionary_encode: an input with a validity bitmap needs a dictionary validity bitmap in encode mode");
+  if ((reinterpret_cast<uintptr_t>(indices) & 3) || (reinterpret_cast<uintptr_t>(indices_valid) & 3) || (reinterpret_cast<uintptr_t>(dict_valid) & 3))
+    AG_FAIL(AG_ERR_INVALID, "dictionary_encode: indices and bitmaps must be 4-byte aligned");
+  if (n >= (1ll << 31)) AG_FAIL(AG_ERR_NOT_IMPLEMENTED, "dictionary_encode: more than 2^31-1 rows per call");
+  switch (bit_width) {
+    case 8: return dictionary_encode_t<uint8_t>(vals, valid, off, n, null_encoding, indices, indices_valid, dict, dict_valid, dict_capacity, d_counts, st);
+    case 16: return dictionary_encode_t<uint16_t>(vals, valid, off, n, null_encoding, indices, indices_valid, dict, dict_valid, dict_capacity, d_counts, st);
+    case 32: return dictionary_encode_t<uint32_t>(vals, valid, off, n, null_encoding, indices, indices_valid, dict, dict_valid, dict_capacity, d_counts, st);
+    case 64: return dictionary_encode_t<unsigned long long>(vals, valid, off, n, null_encoding, indices, indices_valid, dict, dict_valid, dict_capacity, d_counts, st);
+    default: AG_FAIL(AG_ERR_NOT_IMPLEMENTED, "dictionary_encode: fixed-width values of 1/2/4/8 bytes only (got %d bits)", bit_width);
   }
 }
 
@@ -528,4 +809,12 @@ extern "C" ag_status ag_unique_dev(int bit_width, const void* d_vals, const uint
                                    uint8_t* d_out_valid, int64_t capacity, int64_t* d_out_len, ag_stream_t s) {
   AG_TRY(ensure_init());
   return unique_dev(bit_width, d_vals, d_valid, offset, n, d_out, d_out_valid, capacity, d_out_len, resolve_stream(s));
+}
+
+extern "C" ag_status ag_dictionary_encode_dev(int bit_width, const void* d_vals, const uint8_t* d_valid, int64_t offset, int64_t n, int null_encoding,
+                                              int32_t* d_indices, uint8_t* d_indices_valid, void* d_dict, uint8_t* d_dict_valid,
+                                              int64_t dict_capacity, int64_t* d_counts, ag_stream_t s) {
+  AG_TRY(ensure_init());
+  return dictionary_encode_dev(bit_width, d_vals, d_valid, offset, n, null_encoding, d_indices, d_indices_valid, d_dict, d_dict_valid,
+                               dict_capacity, d_counts, resolve_stream(s));
 }

@@ -49,6 +49,8 @@ ag_status is_in_dev(int bit_width, const void* vals, const uint8_t* valid, int64
                     int64_t set_off, int64_t set_n, int null_behavior, uint8_t* out_data, uint8_t* out_valid, int64_t* d_null_count, cudaStream_t st);
 ag_status unique_dev(int bit_width, const void* vals, const uint8_t* valid, int64_t off, int64_t n, void* out, uint8_t* out_valid, int64_t capacity,
                      int64_t* d_out_len, cudaStream_t st);
+ag_status dictionary_encode_dev(int bit_width, const void* vals, const uint8_t* valid, int64_t off, int64_t n, int null_encoding, int32_t* indices,
+                                uint8_t* indices_valid, void* dict, uint8_t* dict_valid, int64_t dict_capacity, int64_t* d_counts, cudaStream_t st);
 ag_status sort_indices_dev(int type, const void* vals, const uint8_t* valid, int64_t voff, int64_t n, int order, int null_placement,
                            uint64_t* d_out, int64_t* nulls_out, int64_t* nans_out, cudaStream_t st);
 ag_status take_primitive_dev(int bit_width, const void* vals, const uint8_t* vvalid, int64_t voff, int64_t vlen, int idx_width, int idx_signed,
@@ -905,6 +907,49 @@ ag_status ag_unique(int bit_width, const void* vals, const uint8_t* valid, int64
   }
   AG_TRY(sync(cs));
   *out_len = len;
+  return AG_OK;
+}
+
+ag_status ag_dictionary_encode(int bit_width, const void* vals, const uint8_t* valid, int64_t offset, int64_t n, int null_encoding, int32_t* indices,
+                               uint8_t* indices_valid, void* dict, uint8_t* dict_valid, int64_t* dict_len, int64_t* index_nulls) {
+  AG_TRY(ensure_init());
+  if (!dict_len) AG_FAIL(AG_ERR_INVALID, "dictionary_encode: NULL dict_len");
+  *dict_len = 0;
+  if (index_nulls) *index_nulls = 0;
+  if (bit_width != 8 && bit_width != 16 && bit_width != 32 && bit_width != 64) AG_FAIL(AG_ERR_NOT_IMPLEMENTED, "dictionary_encode: fixed-width values of 1/2/4/8 bytes only");
+  if (n < 0 || offset < 0) AG_FAIL(AG_ERR_INVALID, "dictionary_encode: negative length or offset");
+  if (null_encoding != AG_NULL_ENCODING_MASK && null_encoding != AG_NULL_ENCODING_ENCODE)
+    AG_FAIL(AG_ERR_INVALID, "dictionary_encode: invalid null encoding behavior %d", null_encoding);
+  if (n == 0) return AG_OK;
+  if (!vals || !indices || !dict) AG_FAIL(AG_ERR_INVALID, "dictionary_encode: NULL values / indices / dictionary");
+  if (valid && null_encoding == AG_NULL_ENCODING_MASK && !indices_valid)
+    AG_FAIL(AG_ERR_INVALID, "dictionary_encode: an input with a validity bitmap needs an indices validity bitmap in mask mode");
+  if (valid && null_encoding == AG_NULL_ENCODING_ENCODE && !dict_valid)
+    AG_FAIL(AG_ERR_INVALID, "dictionary_encode: an input with a validity bitmap needs a dictionary validity bitmap in encode mode");
+  const int w = bit_width / 8;
+  CallStream cs; AG_TRY(cs.acquire());
+  Temps t(cs);
+  void *dv, *ddict; uint8_t *dvv, *div = nullptr, *ddv = nullptr; int64_t ov; int32_t* didx; int64_t* d_counts;
+  AG_TRY(t.alloc(&dv, (size_t)n * w));
+  AG_TRY(h2d(dv, (const char*)vals + offset * w, (size_t)n * w, cs));
+  AG_TRY(upload_bitmap(t, valid, offset, n, &dvv, &ov));
+  AG_TRY(t.alloc_t(&didx, (size_t)n * 4));
+  AG_TRY(t.alloc(&ddict, (size_t)n * w));
+  const size_t bm = (size_t)((n + 31) / 32) * 4;
+  if (indices_valid) AG_TRY(t.alloc_t(&div, bm));
+  if (dict_valid) AG_TRY(t.alloc_t(&ddv, bm));
+  AG_TRY(t.alloc_t(&d_counts, 16));
+  AG_TRY(dictionary_encode_dev(bit_width, (const char*)dv - ov * w, dvv, ov, n, null_encoding, didx, div, ddict, ddv, n, d_counts, cs));
+  int64_t counts[2] = {0, 0};
+  AG_TRY(d2h(counts, d_counts, 16, cs));
+  AG_TRY(sync(cs));
+  AG_TRY(d2h(indices, didx, (size_t)n * 4, cs));
+  if (div) AG_TRY(d2h(indices_valid, div, (size_t)((n + 7) / 8), cs));
+  AG_TRY(d2h(dict, ddict, (size_t)counts[0] * w, cs));
+  if (ddv) AG_TRY(d2h(dict_valid, ddv, (size_t)((counts[0] + 7) / 8), cs));
+  AG_TRY(sync(cs));
+  *dict_len = counts[0];
+  if (index_nulls) *index_nulls = counts[1];
   return AG_OK;
 }
 

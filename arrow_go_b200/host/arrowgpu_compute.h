@@ -33,9 +33,10 @@ namespace arrowgpu {
 // ---- arrow.Type (arrow/datatype.go:36-72) -----------------------------------------------
 enum class Type : int {
   NA = 0, BOOL = 1, UINT8 = 2, INT8 = 3, UINT16 = 4, INT16 = 5, UINT32 = 6, INT32 = 7,
-  UINT64 = 8, INT64 = 9, FLOAT16 = 10, FLOAT32 = 11, FLOAT64 = 12
+  UINT64 = 8, INT64 = 9, FLOAT16 = 10, FLOAT32 = 11, FLOAT64 = 12,
+  DICTIONARY = 29  // int32 indices + a dictionary of the value type (dictionary_encode's output)
 };
-int BitWidth(Type t);  // 1 for BOOL
+int BitWidth(Type t);  // 1 for BOOL; 0 for DICTIONARY: no kernel may take a dictionary array for its int32 indices
 const char* TypeName(Type t);
 bool IsInteger(Type t);
 bool IsSignedInteger(Type t);
@@ -77,24 +78,25 @@ class Buffer {
   std::function<void()> on_release_;
 };
 
-// arrow.ArrayData for primitive / boolean arrays (arrow/array/data.go:30-42)
+// arrow.ArrayData for primitive / boolean / dictionary arrays (arrow/array/data.go:30-42)
 struct ArrayData {
   Type type = Type::NA;
   int64_t length = 0;
   int64_t null_count = 0;  // kUnknownNullCount allowed
   int64_t offset = 0;
-  std::shared_ptr<Buffer> buffers[2];  // [0] validity bitmap (may be null), [1] values / boolean data
+  std::shared_ptr<Buffer> buffers[2];  // [0] validity bitmap (may be null), [1] values / boolean data (DICTIONARY: int32 indices)
+  std::shared_ptr<ArrayData> dictionary;  // DICTIONARY only: the values the indices point at (its type is the value type)
   std::shared_ptr<ArrayData> Slice(int64_t off, int64_t len) const;  // array.NewSlice semantics
   // validity (LSB-first bitmap, `offset` applies) may be NULL; values must hold (offset+length) elements
   static Status FromHost(Type type, int64_t length, int64_t offset, const uint8_t* validity, const void* values,
                          int64_t null_count, std::shared_ptr<ArrayData>* out);
   // Copies the logical [0,length) range out: values (length elements, or ceil(length/8) bytes for BOOL,
-  // bit 0 = element 0) and validity (ceil(length/8) bytes; all ones when there is no bitmap).
+  // bit 0 = element 0; the int32 indices for DICTIONARY) and validity (ceil(length/8) bytes; all ones when there is no bitmap).
   Status ToHost(void* values, uint8_t* validity, int64_t* null_count) const;
   // Arrow C Device Data Interface (include/arrowgpu_cdata.h).  Export shares the buffers: the exported
   // struct keeps them alive until the consumer calls release.  Import takes ownership of `in`
   // (moves it; in->array.release is called when the last buffer reference is dropped) and makes the
-  // default stream wait on its sync_event.
+  // default stream wait on its sync_event.  Dictionary arrays are not exported (ErrNotImplemented).
   Status ExportDevice(struct ArrowDeviceArray* out, struct ArrowSchema* out_schema) const;
   static Status ImportDevice(struct ArrowDeviceArray* in, const struct ArrowSchema* schema, std::shared_ptr<ArrayData>* out);
 };
@@ -262,6 +264,12 @@ struct SetLookupOptions : FunctionOptions {                   // compute/scalar_
   const char* TypeName() const override { return "SetLookupOptions"; }
 };
 
+enum NullEncodingBehavior { NullEncodingMask = 0, NullEncodingEncode = 1 };   // kernels/vector_hash.go:83-91
+struct DictionaryEncodeOptions : FunctionOptions {                           // :93-98
+  NullEncodingBehavior NullEncoding = NullEncodingMask;
+  const char* TypeName() const override { return "DictionaryEncodeOptions"; }
+};
+
 enum class FuncKind { SCALAR, VECTOR, META };  // functions.go FuncScalar / FuncVector / FuncMeta
 
 class FunctionRegistry;
@@ -357,6 +365,9 @@ Status Take(const ExecCtx& ctx, const TakeOptions& opts, const Datum& values, co
 Status SortIndices(const ExecCtx& ctx, const Datum& input, const SortOptions& opts, Datum* out);
 Status Unique(const ExecCtx& ctx, const Datum& values, Datum* out);
 Status IsIn(const ExecCtx& ctx, const SetLookupOptions& opts, const Datum& values, Datum* out);
+// compute.DictionaryEncode (vector_hash.go): a DICTIONARY array (one per chunk of a chunked input, all sharing one
+// dictionary) of the 10 numeric types; a dictionary input is returned unchanged
+Status DictionaryEncode(const ExecCtx& ctx, const DictionaryEncodeOptions& opts, const Datum& values, Datum* out);
 
 // ---- executor internals exposed for tests (exec_internals_test.go exercises the same pieces) ----
 struct SpanPiece { int64_t pos; int64_t len; std::vector<int> chunk_index; std::vector<int64_t> chunk_pos; };

@@ -134,6 +134,19 @@ int agx_is_in(agx_datum* d, agx_datum* value_set, int null_behavior, agx_datum**
   *out = new agx_datum{res};
   return AG_OK;
 }
+// compute.DictionaryEncode(DictionaryEncodeOptions{NullEncoding}); agx_dictionary: the dictionary of a dictionary array
+int agx_dictionary_encode(agx_datum* d, int null_encoding, agx_datum** out) {
+  DictionaryEncodeOptions o; o.NullEncoding = (NullEncodingBehavior)null_encoding;
+  ExecCtx ctx; Datum res;
+  AGX_TRY(DictionaryEncode(ctx, o, d->d, &res));
+  *out = new agx_datum{res};
+  return AG_OK;
+}
+int agx_dictionary(agx_datum* d, agx_datum** out) {
+  if (d->d.kind != DatumKind::ARRAY || !d->d.array->dictionary) return fail(Status::Invalid("dictionary: not a dictionary array"));
+  *out = new agx_datum{Datum(d->d.array->dictionary)};
+  return AG_OK;
+}
 int agx_scalar_value(agx_datum* d, int* valid, void* value8) {
   if (d->d.kind != DatumKind::SCALAR) return fail(Status::Invalid("scalar_value: not a scalar"));
   *valid = d->d.scalar->valid ? 1 : 0;

@@ -16,12 +16,13 @@ int BitWidth(Type t) {
     case Type::UINT16: case Type::INT16: case Type::FLOAT16: return 16;
     case Type::UINT32: case Type::INT32: case Type::FLOAT32: return 32;
     case Type::UINT64: case Type::INT64: case Type::FLOAT64: return 64;
-    default: return 0;
+    default: return 0;  // DICTIONARY included: its int32 indices are not values of the array's type
   }
 }
 const char* TypeName(Type t) {
   static const char* names[] = {"null", "bool", "uint8", "int8", "uint16", "int16", "uint32", "int32", "uint64", "int64", "float16", "float32", "float64"};
   const int i = (int)t;
+  if (t == Type::DICTIONARY) return "dictionary";
   return (i >= 0 && i <= 12) ? names[i] : "unknown";
 }
 bool IsSignedInteger(Type t) { return t == Type::INT8 || t == Type::INT16 || t == Type::INT32 || t == Type::INT64; }
@@ -97,6 +98,7 @@ void ReleaseExportedBuffers(void* opaque) { delete static_cast<ExportedBuffers*>
 }  // namespace
 
 Status ArrayData::ExportDevice(struct ArrowDeviceArray* out, struct ArrowSchema* out_schema) const {
+  if (type == Type::DICTIONARY) return Status::NotImplemented("export: dictionary arrays are not exported through the C Device Data Interface");
   auto* keep = new ExportedBuffers{{buffers[0], buffers[1]}};
   const int rc = ag_export_device_array((int)type, length, null_count, offset, buffers[0] ? buffers[0]->data() : nullptr,
                                         buffers[1] ? buffers[1]->data() : nullptr, ReleaseExportedBuffers, keep, nullptr, out, out_schema);
@@ -145,7 +147,7 @@ Status ArrayData::FromHost(Type type, int64_t length, int64_t offset, const uint
 
 Status ArrayData::ToHost(void* values, uint8_t* validity, int64_t* null_count_out) const {
   if (length == 0) { if (null_count_out) *null_count_out = 0; return Status::OK(); }
-  const int w = BitWidth(type);
+  const int w = type == Type::DICTIONARY ? 32 : BitWidth(type);
   if (values) {
     if (type == Type::BOOL) {
       // re-base to bit 0 on the device, then copy
@@ -472,11 +474,19 @@ Status VectorFunction::DispatchExact(const std::vector<Type>& types, const exec:
 }
 
 // ---------------------------------------------------------------- scalar executor ---------
+// A DICTIONARY array is its int32 indices plus a dictionary: no kernel of this layer decodes it, and none may read the
+// indices as values of the array's type.
+static Status RejectDictionaries(const std::string& fn, const std::vector<Datum>& args) {
+  for (auto& a : args)
+    if (a.kind != DatumKind::NONE && a.kind != DatumKind::SCALAR && a.type() == Type::DICTIONARY)
+      return Status::NotImplemented("function '" + fn + "' does not take dictionary arrays");
+  return Status::OK();
+}
 static Status CheckArgs(const Function& fn, const std::vector<Datum>& args) {
   if ((int)args.size() != fn.Arity())
     return Status::Invalid("function '" + fn.Name() + "' accepts " + std::to_string(fn.Arity()) + " arguments but " + std::to_string(args.size()) + " passed");
   for (auto& a : args) if (a.kind == DatumKind::NONE) return Status::Invalid("tried executing function with non-value type");  // checkAllIsValue
-  return Status::OK();
+  return RejectDictionaries(fn.Name(), args);
 }
 
 namespace {
@@ -1370,6 +1380,7 @@ std::shared_ptr<ScalarFunction> MakeBool(const std::string& name, exec::ArrayKer
 }
 
 Status ConcatenateChunks(const ChunkedArray& c, std::shared_ptr<ArrayData>* out);
+Status DictionaryEncodeImpl(const DictionaryEncodeOptions& opts, const Datum& values, Datum* out);
 
 }  // namespace
 
@@ -1470,6 +1481,7 @@ FunctionRegistry* GetFunctionRegistry() {
       const auto* co = dynamic_cast<const CastOptions*>(fo);
       if (!co || co->ToType == Type::NA) return Status::Invalid("cast requires that options be passed with a ToType");
       if (args.size() != 1 || args[0].kind == DatumKind::NONE) return Status::Invalid("cast takes one value argument");
+      RETURN_NOT_OK(RejectDictionaries("cast", args));
       if (args[0].type() == co->ToType) { *out = args[0]; return Status::OK(); }
       const char* fname = CastFunctionName(co->ToType);
       FunctionRegistry* r = ctx.Registry ? ctx.Registry : GetFunctionRegistry();
@@ -1506,6 +1518,11 @@ FunctionRegistry* GetFunctionRegistry() {
       if (!so) return Status::Invalid("is_in requires SetLookupOptions");
       if (args.size() != 1) return Status::Invalid("is_in takes one argument");
       return IsIn(ctx, *so, args[0], out);
+    }), false);
+    reg->AddFunction(std::make_shared<MetaFunction>("dictionary_encode", 1, [](const ExecCtx& ctx, const FunctionOptions* fo, const std::vector<Datum>& args, Datum* out) -> Status {
+      const auto* o = dynamic_cast<const DictionaryEncodeOptions*>(fo);
+      if (args.size() != 1) return Status::Invalid("dictionary_encode takes one argument");
+      return DictionaryEncodeImpl(o ? *o : DictionaryEncodeOptions(), args[0], out);
     }), false);
     // vector_cumulative.go:75-93
     reg->AddFunction(MakeCumulative("cumulative_sum", false), false);
@@ -1545,6 +1562,7 @@ FunctionRegistry* GetFunctionRegistry() {
     reg->AddFunction(std::make_shared<MetaFunction>("take", 2, [](const ExecCtx& ctx, const FunctionOptions* opts, const std::vector<Datum>& args, Datum* out) -> Status {
       // takeMetaFunc, selection.go:93-114 -> takeArrayImpl :206-244 / takeChunkedImpl :246-300
       if (args.size() != 2) return Status::Invalid("take takes 2 arguments");
+      RETURN_NOT_OK(RejectDictionaries("take", args));
       if (args[1].kind != DatumKind::ARRAY && args[1].kind != DatumKind::CHUNKED) return Status::NotImplemented("unsupported types for take operation");
       Datum values = args[0];
       const bool values_chunked = values.kind == DatumKind::CHUNKED;
@@ -1600,6 +1618,62 @@ Status ConcatenateChunks(const ChunkedArray& c, std::shared_ptr<ArrayData>* out)
   }
   d->null_count = any_nulls ? kUnknownNullCount : 0;
   *out = d;
+  return Status::OK();
+}
+
+// dictionaryEncodeAction (kernels/vector_hash.go:144-241) over doAppendNumeric (:359-385): the chunks of a chunked input
+// are concatenated on the device and encoded in one call, so every chunk's indices point into one dictionary
+// (dictionaryEncodeFinalize :854-872); the output chunks are zero-copy slices of one indices buffer.
+Status DictionaryEncodeImpl(const DictionaryEncodeOptions& opts, const Datum& values, Datum* out) {
+  if (opts.NullEncoding != NullEncodingMask && opts.NullEncoding != NullEncodingEncode)
+    return Status::Invalid("invalid null encoding behavior " + std::to_string((int)opts.NullEncoding));  // :103-104
+  if (values.kind != DatumKind::ARRAY && values.kind != DatumKind::CHUNKED) return Status::NotImplemented("dictionary_encode takes an array or a chunked array");
+  if (values.type() == Type::DICTIONARY) { *out = values; return Status::OK(); }  // dictionaryEncodeIdentity :473-500
+  const Type t = values.type();
+  if (!IsNumeric(t)) return Status::NotImplemented(std::string("dictionary_encode: unsupported type ") + TypeName(t));
+  const int bw = BitWidth(t);
+  std::shared_ptr<ArrayData> a;
+  if (values.kind == DatumKind::ARRAY) a = values.array;
+  else if (values.chunked->chunks.size() == 1) a = values.chunked->chunks[0];
+  else if (values.chunked->chunks.empty()) { a = std::make_shared<ArrayData>(); a->type = t; }
+  else RETURN_NOT_OK(ConcatenateChunks(*values.chunked, &a));
+  if (a->length >= (1ll << 31)) return Status::NotImplemented("dictionary_encode: more than 2^31-1 rows per call");
+  const bool encode = opts.NullEncoding == NullEncodingEncode;
+  const bool has_valid = a->buffers[0] && a->null_count != 0;
+  const int64_t n = a->length;
+  std::shared_ptr<Buffer> idx, idx_valid, dict, dict_valid, counts;
+  RETURN_NOT_OK(Buffer::Allocate(std::max<int64_t>(n, 1) * 4, &idx));
+  RETURN_NOT_OK(Buffer::Allocate(std::max<int64_t>(n, 1) * (bw / 8), &dict));
+  const int64_t bm = ((n + 31) / 32) * 4 + 4;
+  if (has_valid && !encode) RETURN_NOT_OK(Buffer::Allocate(bm, &idx_valid));
+  if (has_valid && encode) RETURN_NOT_OK(Buffer::Allocate(bm, &dict_valid));
+  RETURN_NOT_OK(Buffer::Allocate(16, &counts));
+  NATIVE(ag_dictionary_encode_dev(bw, a->buffers[1] ? a->buffers[1]->data() : nullptr, has_valid ? a->buffers[0]->data() : nullptr, a->offset, n,
+                                  (int)opts.NullEncoding, (int32_t*)idx->data(), idx_valid ? idx_valid->data() : nullptr, dict->data(),
+                                  dict_valid ? dict_valid->data() : nullptr, n, (int64_t*)counts->data(), nullptr));
+  int64_t c[2] = {0, 0};
+  RETURN_NOT_OK(counts->ToHost(c, 16));
+  auto d = std::make_shared<ArrayData>();
+  d->type = t; d->length = c[0];
+  d->buffers[1] = dict;
+  d->buffers[0] = dict_valid;
+  d->null_count = !dict_valid ? 0 : (a->null_count > 0 ? 1 : kUnknownNullCount);  // the one null entry, when the input has a null
+  auto r = std::make_shared<ArrayData>();
+  r->type = Type::DICTIONARY; r->length = n;
+  r->buffers[1] = idx;
+  r->buffers[0] = idx_valid;
+  r->null_count = idx_valid ? c[1] : 0;
+  r->dictionary = d;
+  if (values.kind == DatumKind::ARRAY) { *out = Datum(r); return Status::OK(); }
+  auto res = std::make_shared<ChunkedArray>();
+  res->type = Type::DICTIONARY;
+  int64_t pos = 0;
+  for (auto& ch : values.chunked->chunks) {
+    res->chunks.push_back(r->Slice(pos, ch->length));
+    pos += ch->length;
+  }
+  res->length = pos;
+  *out = Datum(res);
   return Status::OK();
 }
 }  // namespace
@@ -1695,6 +1769,10 @@ Status IsIn(const ExecCtx& ctx, const SetLookupOptions& opts, const Datum& value
   int64_t nulls = 0;
   RETURN_NOT_OK(cnt->ToHost(&nulls, 8));
   return MakeOut(Type::BOOL, a->length, data, nulls ? valid : nullptr, nulls, out);
+}
+
+Status DictionaryEncode(const ExecCtx& ctx, const DictionaryEncodeOptions& opts, const Datum& values, Datum* out) {
+  return CallFunction(ctx, "dictionary_encode", &opts, {values}, out);
 }
 
 Status Filter(const ExecCtx& ctx, const Datum& values, const Datum& filter, const FilterOptions& opts, Datum* out) {

@@ -221,10 +221,146 @@ func sortOneColumn(ctx context.Context, col arrow.ArrayData, key compute.SortKey
 	return &compute.ArrayDatum{Value: out}, nil
 }
 
-// registerLookupSort adds is_in, unique and sort_indices to a registry built by NewRegistry.
+// ---- dictionary_encode (vector_hash.go:105-125, kernels/vector_hash.go:83-241,359-385,854-925) -----------------------
+//
+// Like unique, ag_dictionary_encode needs the whole column at once (a value's dictionary position is the rank of its
+// first row), so the kernel is not chunk-wise: a chunked input is concatenated, encoded in one call, and its indices are
+// split back into the input's chunk lengths.  The dictionary waits in the kernel state until Finalize attaches it to
+// every result (dictionaryEncodeFinalize :854-872), so all chunks share one dictionary.  Dictionary inputs (the
+// identity kernel) and every non-numeric type go to the parent registry.
+
+type dictEncodeState struct {
+	nullEncoding C.int // NullEncodingMask 0 / NullEncodingEncode 1 (= AG_NULL_ENCODING_*)
+	dict         arrow.ArrayData
+}
+
+// initDictEncode restates parseDictionaryEncodeOptions (kernels/vector_hash.go:811-829).
+func initDictEncode(_ *exec.KernelCtx, args exec.KernelInitArgs) (exec.KernelState, error) {
+	opts := compute.DictionaryEncodeOptions{}
+	switch o := args.Options.(type) {
+	case nil:
+	case compute.DictionaryEncodeOptions:
+		opts = o
+	case *compute.DictionaryEncodeOptions:
+		if o != nil {
+			opts = *o
+		}
+	default:
+		return nil, fmt.Errorf("%w: expected DictionaryEncodeOptions, got %T", arrow.ErrInvalid, args.Options)
+	}
+	if opts.NullEncoding != compute.NullEncodingMask && opts.NullEncoding != compute.NullEncodingEncode {
+		return nil, fmt.Errorf("%w: invalid null encoding behavior %d", arrow.ErrInvalid, opts.NullEncoding)
+	}
+	return &dictEncodeState{nullEncoding: C.int(opts.NullEncoding)}, nil
+}
+
+func dictEncodeExec(ctx *exec.KernelCtx, batch *exec.ExecSpan, out *exec.ExecResult) error {
+	st := ctx.State.(*dictEncodeState)
+	in := &batch.Values[0].Array
+	bw := in.Type.(arrow.FixedWidthDataType).BitWidth()
+	mask := st.nullEncoding == C.AG_NULL_ENCODING_MASK
+	preallocate(ctx, in.Len, 32, in.MayHaveNulls() && mask, out)
+	dictVals := ctx.Allocate(int(in.Len) * (bw / 8)) // n entries are always enough; the length is trimmed below
+	var dictValid *memory.Buffer
+	var dictValidBytes []byte
+	if in.MayHaveNulls() && !mask {
+		dictValid = ctx.AllocateBitmap(in.Len)
+		dictValidBytes = dictValid.Bytes()
+	}
+	var dictLen, nulls C.int64_t
+	err := check(C.ag_dictionary_encode(C.int(bw), base0(in.Buffers[1].Buf), validityOf(in), C.int64_t(in.Offset), C.int64_t(in.Len),
+		st.nullEncoding, (*C.int32_t)(base0(out.Buffers[1].Buf)), bitmap(out.Buffers[0].Buf), base0(dictVals.Bytes()), bitmap(dictValidBytes),
+		&dictLen, &nulls))
+	if err != nil {
+		dictVals.Release()
+		if dictValid != nil {
+			dictValid.Release()
+		}
+		return err
+	}
+	out.Nulls = int64(nulls)
+	dictNulls := 0
+	if dictValid != nil {
+		dictNulls = array.UnknownNullCount
+	}
+	if st.dict != nil {
+		st.dict.Release()
+	}
+	st.dict = array.NewData(in.Type, int(dictLen), []*memory.Buffer{dictValid, dictVals}, nil, dictNulls, 0)
+	dictVals.Release() // NewData retained them
+	if dictValid != nil {
+		dictValid.Release()
+	}
+	return nil
+}
+
+func dictEncodeChunked(ctx *exec.KernelCtx, cols []*arrow.Chunked, out *exec.ExecResult) ([]*exec.ExecResult, error) {
+	arr, err := array.Concatenate(cols[0].Chunks(), exec.GetAllocator(ctx.Ctx))
+	if err != nil {
+		return nil, err
+	}
+	defer arr.Release()
+	span := exec.ExecSpan{Len: int64(arr.Len()), Values: make([]exec.ExecValue, 1)}
+	span.Values[0].Array.SetMembers(arr.Data())
+	if err := dictEncodeExec(ctx, &span, out); err != nil {
+		return nil, err
+	}
+	whole := out.MakeData()
+	defer whole.Release()
+	out.Release() // the chunks below hold their own references
+	results := make([]*exec.ExecResult, 0, len(cols[0].Chunks()))
+	pos := int64(0)
+	for _, ch := range cols[0].Chunks() {
+		part := array.NewSliceData(whole, pos, pos+int64(ch.Len()))
+		r := &exec.ExecResult{}
+		r.TakeOwnership(part)
+		part.Release()
+		results = append(results, r)
+		pos += int64(ch.Len())
+	}
+	return results, nil
+}
+
+func dictEncodeFinalize(ctx *exec.KernelCtx, results []*exec.ArraySpan) ([]*exec.ArraySpan, error) {
+	st := ctx.State.(*dictEncodeState)
+	if st.dict == nil {
+		return results, nil
+	}
+	for _, r := range results {
+		var d exec.ArraySpan
+		d.TakeOwnership(st.dict)
+		r.SetDictionary(&d)
+	}
+	st.dict.Release()
+	st.dict = nil
+	return results, nil
+}
+
+func dictEncodeFunction() *compute.VectorFunction {
+	fn := compute.NewVectorFunction("dictionary_encode", compute.Unary(), compute.EmptyFuncDoc)
+	outType := exec.NewComputedOutputType(func(_ *exec.KernelCtx, args []arrow.DataType) (arrow.DataType, error) {
+		return &arrow.DictionaryType{IndexType: arrow.PrimitiveTypes.Int32, ValueType: args[0]}, nil
+	})
+	for _, ty := range numericTypes {
+		k := exec.NewVectorKernel([]exec.InputType{exec.NewExactInput(ty)}, outType, dictEncodeExec, initDictEncode)
+		k.CanExecuteChunkWise = false
+		k.OutputChunked = true
+		k.ExecChunked = dictEncodeChunked
+		k.Finalize = dictEncodeFinalize
+		k.NullHandling = exec.NullComputedNoPrealloc
+		k.MemAlloc = exec.MemNoPrealloc
+		if err := fn.AddKernel(k); err != nil {
+			panic(err)
+		}
+	}
+	return fn
+}
+
+// registerLookupSort adds is_in, unique, dictionary_encode and sort_indices to a registry built by NewRegistry.
 func registerLookupSort(reg, parent compute.FunctionRegistry) {
 	addScalar(reg, parent, isInFunction())
 	addVector(reg, parent, uniqueFunction())
+	addVector(reg, parent, dictEncodeFunction())
 	p, _ := parent.GetFunction("sort_indices")
 	reg.AddFunction(sortIndicesFunction(p), true)
 }

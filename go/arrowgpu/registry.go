@@ -213,7 +213,7 @@ func NewRegistry() compute.FunctionRegistry {
 	}
 	addVector(reg, parent, filterFn)
 	addVector(reg, parent, takeFn)
-	registerLookupSort(reg, parent) // is_in, unique, sort_indices (lookup_sort.go)
+	registerLookupSort(reg, parent) // is_in, unique, dictionary_encode, sort_indices (lookup_sort.go)
 	return reg
 }
 

@@ -527,6 +527,33 @@ ag_status ag_unique_dev(int bit_width, const void* d_vals, const uint8_t* d_vali
 ag_status ag_unique_set_policy(int64_t small_rows, int64_t small_slots);
 
 /* ================================================================================= *
+ * dictionary_encode for fixed-width values of 1/2/4/8 bytes — kernels/vector_hash.go:83-141
+ *   (NullEncodingBehavior, DictionaryEncodeOptions), :144-241 (dictionaryEncodeAction), :359-385
+ *   (doAppendNumeric), :854-872 (dictionaryEncodeFinalize).  Same key equality and table policy as unique
+ *   (raw bytes; ag_unique_set_policy).
+ *   dict: the distinct values in order of first appearance; indices: one int32 per row = its value's position.
+ *   AG_NULL_ENCODING_MASK  : a null row gets index 0 and a null in the indices (indices_valid, bit offset 0);
+ *                            the dictionary has no null entry.
+ *   AG_NULL_ENCODING_ENCODE: the nulls share one dictionary entry placed where the first null appears (its
+ *                            dict_valid bit cleared, its value bytes 0); the indices have no nulls.
+ *   Any other null_encoding is AG_ERR_INVALID.  An input with a validity bitmap needs indices_valid in mask mode
+ *   and dict_valid in encode mode.  indices / indices_valid / dict_valid: 4-byte aligned, bit offset 0; a given
+ *   indices_valid is fully written (ceil(n/32) words).  `offset` is the element offset into both the values
+ *   buffer and the validity bitmap.  n < 2^31 rows per call.
+ *   Host flavour: dict (and dict_valid) need room for n entries; *dict_len / *index_nulls receive the counts.
+ *   Device flavour: d_counts[0] = dictionary length, d_counts[1] = null count of the indices; entries past
+ *   dict_capacity are dropped (d_counts[0] still receives the full length, so a truncation is detectable).
+ * ================================================================================= */
+#define AG_NULL_ENCODING_MASK   0
+#define AG_NULL_ENCODING_ENCODE 1
+ag_status ag_dictionary_encode(int bit_width, const void* vals, const uint8_t* valid, int64_t offset, int64_t n,
+                               int null_encoding, int32_t* indices, uint8_t* indices_valid, void* dict,
+                               uint8_t* dict_valid, int64_t* dict_len, int64_t* index_nulls);
+ag_status ag_dictionary_encode_dev(int bit_width, const void* d_vals, const uint8_t* d_valid, int64_t offset, int64_t n,
+                                   int null_encoding, int32_t* d_indices, uint8_t* d_indices_valid, void* d_dict,
+                                   uint8_t* d_dict_valid, int64_t dict_capacity, int64_t* d_counts, ag_stream_t s);
+
+/* ================================================================================= *
  * sort_indices, one fixed-width column (SURVEY 8f rank 3) — replaces kernels.SortIndices for a single
  *   key (vector_sort.go:385-481, vector_sort_internal.go:36-150,250-300): a STABLE permutation of
  *   0..n-1 as uint64 row indices,
